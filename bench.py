@@ -22,6 +22,9 @@ are processed in order because scan t+1 reads the prior written by scan t.
 `--impl reference` times the reference's own CPU implementation on all host cores, one independent stream per core:
 oracle/_ref (the unmodified reference sources compiled on CPU stand-ins, cpu_baseline.kind = "reference") when the
 prebuilt library is there, else the oracle port.
+
+`--dump-outputs DIR` writes what the last timed step computed for a fixed sample of streams (dump_outputs) as .npy files;
+the inputs depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -240,7 +243,7 @@ def reference_arm(args, rank, world):
         for th in ths:
             th.join()
 
-    steps = min(args.steps, 20)      # a bounded sample: every step is one scan on every core
+    steps = args.steps               # every step is one scan on every core
     for t in range(args.warmup):
         step(t)
     t0 = time.perf_counter()
@@ -264,6 +267,29 @@ def reference_arm(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_STREAMS = 32   # 32 streams x (labels and output order of <= 131072 points + two 300 x 300 layers) in float32: <= 57 MB
+
+
+def dump_outputs(g, out_dir, npts):
+    """What the last timed step handed back, for a fixed seeded sample of the streams: per input point the label, the
+    output order (input index of each output point, gg_get_output) and, per cell, the ground height and confidence
+    that the next scan of the stream reads.  Per-stream arrays are concatenated in the order of streams.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    sample = np.sort(np.random.default_rng(0).choice(g.n_slots, min(DUMP_STREAMS, g.n_slots), replace=False))
+    labels = [g.download_labels(int(npts[b]), slot=int(b)) for b in sample]
+    g.synchronize()
+    order = [g.get_output(slot=int(b))[0] for b in sample]
+    out = {"streams": sample.astype(np.float64),
+           "points_per_stream": np.array([len(v) for v in labels], np.float64),
+           "labels": np.concatenate(labels).astype(np.float32),
+           "output_points_per_stream": np.array([len(v) for v in order], np.float64),
+           "output_order": np.concatenate(order).astype(np.float32),   # indices < 2^24: exact in float32
+           "ground": np.stack([g.layer("ground", int(b)) for b in sample]),
+           "groundpatch": np.stack([g.layer("groundpatch", int(b)) for b in sample])}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def bind_to_gpu_numa_node(torch, local_rank):
@@ -383,7 +409,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip cfg3 / cfg4 / drop-in latency / serialised per-kernel roofline / prior broadcast")
     ap.add_argument("--no-bind", action="store_true", help="do not bind the process to the NUMA node of its GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last of them computed "
+                    "(labels, output order, ground / groundpatch of a fixed sample of streams) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -543,6 +573,8 @@ def main():
     prof = g.profile_read(reset=True)
     g.profile_enable(False)
     value = sum_over_ranks(pts_dev) / (ms_dev * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(g, args.dump_outputs, npts[:, pingpong(tstep[0] - 1, S)])
 
     # ---- end to end through the host-buffer C-ABI call
     e2e = None

@@ -7,6 +7,7 @@ Oracle = reference semantics at thread_count = 1 (see oracle/gg_oracle.cpp heade
 import numpy as np
 import pytest
 
+from golden_util import ReferenceRecord, cloud_values
 from groundgrid_b200 import capi, synth
 from oracle import Oracle
 
@@ -594,37 +595,93 @@ def test_error_codes():
     assert e.value.code == -1
 
 
-@pytest.mark.parametrize("cfg", ["cfg2_300", "cfg3_600", "cfg4_364"])
-def test_cuda_path_against_the_reference_itself(cfg):
-    """The CUDA path against oracle/_ref (the UNMODIFIED reference sources on CPU stand-ins, prebuilt in the container
-    that has /root/reference) at BASELINE.json's full sizes: three scans with a map roll, labels / output order / every
-    layer bit for bit."""
-    from oracle import ref as refmod
+class CudaPath:
+    """The CUDA path, called like the reference: transforms as (quaternion, translation)."""
 
-    if not refmod.available():
-        pytest.skip("oracle/_ref/libgg_ref.so was not shipped")
-    dim, res, scan, maxp = {"cfg2_300": (99.0, 0.33, synth.scan_64, 140000), "cfg3_600": (120.0, 0.2, synth.scan_128, 280000),
-                            "cfg4_364": (120.0, 0.33, synth.scan_4lidar, 520000)}[cfg]
-    g = capi.GroundGridB200(dim, res, n_slots=1, max_points=maxp, full_layers=True)
-    r = refmod.Reference(dim, res)
-    assert g.n == r.n
-    assert np.array_equal(g.layer("expectedPoints"), r.expected_points())
-    g.init_map(0.0, 0.0, 0.0)
-    r.init_map(0.0, 0.0, 0.0)
+    def __init__(self, dim, res, max_points):
+        self.g = capi.GroundGridB200(dim, res, n_slots=1, max_points=max_points, full_layers=True)
+        self.n = self.g.n
+
+    def expected_points(self):
+        return self.g.layer("expectedPoints")
+
+    def init_map(self, x, y, z):
+        self.g.init_map(x, y, z)
+
+    def update(self, x, y, q, t):
+        return self.g.update_pose(x, y, synth.tf2_matrix(q, t))
+
+    def position(self):
+        return self.g.position()
+
+    def filter_cloud(self, pts, org, base_z):
+        labels, index, _ = self.g.filter_cloud(pts, org, base_z, want_index=True)
+        return labels, index
+
+    def layer(self, name):
+        return self.g.layer(name)
+
+    def close(self):
+        self.g.close()
+
+
+class Reference:
+    """The reference, for recording the scenario (needs oracle/_ref)."""
+
+    def __init__(self, dim, res, max_points):
+        from oracle import ref as refmod
+
+        self.r = refmod.Reference(dim, res)
+        self.n = self.r.n
+        self.expected_points, self.init_map, self.position, self.layer = (self.r.expected_points, self.r.init_map,
+                                                                          self.r.position, self.r.layer)
+
+    def update(self, x, y, q, t):
+        return bool(self.r.update(x, y, q, t))
+
+    def filter_cloud(self, pts, org, base_z):
+        return self.r.filter_cloud(pts, org, base_z)[:2]
+
+    def close(self):
+        self.r.close()
+
+
+REFERENCE_CFGS = {"cfg2_300": (99.0, 0.33, synth.scan_64, 140000), "cfg3_600": (120.0, 0.2, synth.scan_128, 280000),
+                  "cfg4_364": (120.0, 0.33, synth.scan_4lidar, 520000)}
+
+
+def full_size_stream(rec, make, cfg):
+    """Three scans with a map roll at one of BASELINE.json's full sizes."""
+    dim, res, scan, maxp = REFERENCE_CFGS[cfg]
+    m = make(dim, res, maxp)
+    rec.check("cells", m.n)
+    rec.check("expectedPoints", m.expected_points())
+    m.init_map(0.0, 0.0, 0.0)
     scene = synth.make_scene(seed=4321, stream_len=20.0, undulation=0.3)
     rng = np.random.default_rng(17)
     for k in range(3):
         ex, ey, yaw = 1.1 * k, -0.45 * k, 0.01 * k
         pts, org = scan(scene, (ex, ey), yaw, seed=700 + k)
         if k:
-            q, t = refmod.base_from_map_qt(ex, ey, yaw, 0.0, pitch=0.02)
-            assert g.update_pose(ex, ey, refmod.tf2_matrix(q, t)) == bool(r.update(ex, ey, q, t))
-            assert np.array_equal(g.position(), r.position())
+            q, t = synth.base_from_map_qt(ex, ey, yaw, 0.0, pitch=0.02)
+            rec.check(f"scan {k}: moved", m.update(ex, ey, q, t))
+            rec.check(f"scan {k}: position", m.position())
             idx = rng.choice(len(pts), 2000, replace=False)
             pts["z"][idx] -= rng.uniform(0.25, 2.0, 2000).astype(np.float32)
-        labels, index, _ = g.filter_cloud(pts, org, 0.0, want_index=True)
-        lab_r, idx_r, _ = r.filter_cloud(pts, org, 0.0)
-        assert np.array_equal(labels, lab_r), f"{cfg} scan {k}: {(labels != lab_r).sum()} labels differ from the reference"
-        assert np.array_equal(index, idx_r)
-        assert_layers_equal(g, r, ("points",) + LIVE + DEAD, f"{cfg} scan {k} vs reference")
-    g.close()
+        rec.check(f"scan {k}: input cloud", cloud_values(pts))
+        labels, index = m.filter_cloud(pts, org, 0.0)
+        rec.check(f"scan {k}: labels", labels)
+        rec.check(f"scan {k}: output order", index)
+        for n in ("points",) + LIVE + DEAD:
+            rec.check(f"scan {k}: layer {n}", m.layer(n))
+    m.close()
+
+
+@pytest.mark.parametrize("cfg", list(REFERENCE_CFGS))
+def test_cuda_path_against_the_reference_itself(cfg):
+    """The CUDA path against oracle/_ref (the UNMODIFIED reference sources on CPU stand-ins; its answers are stored
+    under tests/golden/ref_cuda_*.npz) at BASELINE.json's full sizes: three scans with a map roll, labels / output
+    order / every layer bit for bit."""
+    rec = ReferenceRecord(f"cuda_{cfg}")
+    full_size_stream(rec, CudaPath, cfg)
+    rec.finish()

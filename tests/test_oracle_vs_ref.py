@@ -1,57 +1,61 @@
 """The oracle port (oracle/gg_oracle.cpp) against the REFERENCE ITSELF (oracle/_ref/libgg_ref.so = the unmodified
-/root/reference/src/GroundSegmentation.cpp + GroundGrid.cpp compiled on CPU stand-ins, oracle/build_ref.py).
+reference sources src/GroundSegmentation.cpp + GroundGrid.cpp compiled on CPU stand-ins, oracle/build_ref.py).
 
 This is what pins the oracle: every layer, label, output position and map roll must agree bit for bit at
 thread_count = 1 on the BASELINE.json configurations (cfg1/2: 64 beams, 300x300; cfg3: 128 beams, 600x600;
 cfg4: four LiDARs ~480k points, 364x364), on rolling streams with outliers, and on random geometries / configs.
-The library is built in the container that has /root/reference and travels prebuilt to the GPU box.
+Each test is a scenario run once on the reference (tests/golden/make_reference_records.py) and on the port here:
+the reference's answers are stored under tests/golden/ref_*.npz (golden_util.ReferenceRecord).
 """
-import math
-
 import numpy as np
 import pytest
 
+from golden_util import ReferenceRecord, cloud_values
 from groundgrid_b200 import synth
 from oracle import LAYERS, Oracle
 from oracle import ref as refmod
 
-pytestmark = pytest.mark.skipif(not refmod.available(), reason="oracle/_ref/libgg_ref.so not built (needs /root/reference)")
+
+class Port(Oracle):
+    """The implementation under test, called like the reference: transforms as (quaternion, translation)."""
+
+    def update(self, x, y, q, t):
+        return super().update(x, y, synth.tf2_matrix(q, t))
+
+    def filter_cloud(self, pts, org, base_z):
+        return super().filter_cloud(pts, org, base_z, threads=1, want_cloud=True)
 
 
-def same(a, b):
-    return np.array_equal(a, b, equal_nan=True)
+class Reference(refmod.Reference):
+    """The reference, for recording the scenarios (needs oracle/_ref)."""
+
+    def filter_cloud(self, pts, org, base_z):
+        return super().filter_cloud(pts, org, base_z, want_cloud=True)
 
 
-def assert_layers(o, r, names, ctx):
+def check_layers(rec, m, names, ctx):
     for n in names:
-        a, b = o.layer(n), r.layer(n)
-        if not same(a, b):
-            bad = ~((a == b) | (np.isnan(a) & np.isnan(b)))
-            idx = np.argwhere(bad)[:4]
-            raise AssertionError(f"{ctx}: layer {n}: {bad.sum()} cells differ, e.g. {[(tuple(i), a[tuple(i)], b[tuple(i)]) for i in idx]}")
+        rec.check(f"{ctx}: layer {n}", m.layer(n))
 
 
-def pair(dim, res, **cfg):
-    o, r = Oracle(dim, res), refmod.Reference(dim, res)
-    assert o.n == r.n
+def new_map(rec, make, dim, res, **cfg):
+    m = make(dim, res)
+    rec.check("cells", m.n)
     if cfg:
-        o.set_config(**cfg)
-        r.set_config(**cfg)
-    o.init_map(0.0, 0.0, 0.0)
-    r.init_map(0.0, 0.0, 0.0)
-    assert_layers(o, r, ("points", "ground", "groundpatch", "minGroundHeight", "maxGroundHeight"), "creation")
-    return o, r
+        m.set_config(**cfg)
+    m.init_map(0.0, 0.0, 0.0)
+    check_layers(rec, m, ("points", "ground", "groundpatch", "minGroundHeight", "maxGroundHeight"), "creation")
+    return m
 
 
-def scan_both(o, r, pts, org, base_z, ctx):
-    lo, io, co = o.filter_cloud(pts, org, base_z, threads=1, want_cloud=True)
-    lr, ir, cr = r.filter_cloud(pts, org, base_z, want_cloud=True)
-    assert np.array_equal(lo, lr), f"{ctx}: {(lo != lr).sum()} labels differ"
-    assert np.array_equal(io, ir), f"{ctx}: output order differs"
-    for f in ("x", "y", "z", "intensity", "ring"):  # padding bytes of the records are not part of the value
-        assert np.array_equal(co[f], cr[f]), f"{ctx}: output cloud field {f} differs"
-    assert_layers(o, r, LAYERS, ctx)
-    return lo
+def scan(rec, m, pts, org, base_z, ctx):
+    rec.check(f"{ctx}: input cloud", cloud_values(pts))
+    lab, order, cloud = m.filter_cloud(pts, org, base_z)
+    rec.check(f"{ctx}: labels", lab)
+    rec.check(f"{ctx}: output order", order)
+    rec.check(f"{ctx}: output cloud", cloud_values(cloud))
+    check_layers(rec, m, LAYERS, ctx)
+    return lab
 
 
 def push_below_ground(pts, count, seed):
@@ -60,51 +64,45 @@ def push_below_ground(pts, count, seed):
     pts["z"][idx] -= rng.uniform(0.25, 2.0, count).astype(np.float32)
 
 
-def test_expected_points_table():
+def expected_points_table(rec, make):
     for dim, res in ((99.0, 0.33), (120.0, 0.33), (120.0, 0.2), (33.0, 0.6)):
-        o, r = Oracle(dim, res), refmod.Reference(dim, res)
-        assert o.n == r.n
-        assert np.array_equal(o.expected_points(), r.expected_points())
+        m = make(dim, res)
+        rec.check(f"{dim} m @ {res}: cells", m.n)
+        rec.check(f"{dim} m @ {res}: expected points", m.expected_points())
 
 
-def test_cfg1_cfg2_64_beam_300():
-    """configs[0]/[1]: ~120 k points, 300 x 300 @ 0.33 m; three scans so that the prior is non-trivial."""
-    o, r = pair(99.0, 0.33)
+def cfg1_cfg2_64_beam_300(rec, make):
+    m = new_map(rec, make, 99.0, 0.33)
     scene = synth.make_scene(seed=1234)
     for k in range(3):
         pts, org = synth.scan_64(scene, seed=1234 + k)
         if k == 2:
             push_below_ground(pts, 3000, 5)
-        lab = scan_both(o, r, pts, org, 0.0, f"cfg2 scan {k}")
+        lab = scan(rec, m, pts, org, 0.0, f"cfg2 scan {k}")
     assert (lab == 99).sum() > 10000 and (lab == 49).sum() > 50000
 
 
-def test_cfg3_128_beam_600():
-    """configs[2]: ~240 k points, 600 x 600 @ 0.2 m."""
-    o, r = pair(120.0, 0.2)
-    assert o.n == 600
+def cfg3_128_beam_600(rec, make):
+    m = new_map(rec, make, 120.0, 0.2)
+    assert m.n == 600
     scene = synth.make_scene(seed=77)
     for k in range(2):
         pts, org = synth.scan_128(scene, seed=300 + k)
-        scan_both(o, r, pts, org, 0.0, f"cfg3 scan {k}")
+        scan(rec, m, pts, org, 0.0, f"cfg3 scan {k}")
 
 
-def test_cfg4_four_lidar_364():
-    """configs[3]: four 64-beam sensors, ~480 k points, the reference's own 364 x 364 map."""
-    o, r = pair(120.0, 0.33)
-    assert o.n == 364
+def cfg4_four_lidar_364(rec, make):
+    m = new_map(rec, make, 120.0, 0.33)
+    assert m.n == 364
     scene = synth.make_scene(seed=99)
     for k in range(2):
         pts, org = synth.scan_4lidar(scene, seed=400 + k)
         assert len(pts) > 450000
-        scan_both(o, r, pts, org, 0.0, f"cfg4 scan {k}")
+        scan(rec, m, pts, org, 0.0, f"cfg4 scan {k}")
 
 
-def test_rolling_stream_with_outliers():
-    """12 scans: ego moves, yaws, the base frame is pitched (position-dependent seeding of exposed cells), points
-    pushed below the ground (outlier ray-march against the rolled prior).  Map position, moved flag, the rolled prior and
-    every layer after every scan must agree."""
-    o, r = pair(99.0, 0.33)
+def rolling_stream_with_outliers(rec, make):
+    m = new_map(rec, make, 99.0, 0.33)
     scene = synth.make_scene(seed=1234, stream_len=30.0, undulation=0.3)
     moved_any = 0
     for k in range(12):
@@ -113,41 +111,46 @@ def test_rolling_stream_with_outliers():
         pts, org = synth.scan_64(scene, (ex, ey), yaw, seed=500 + k, az_steps=1024)
         if k:
             q, t = refmod.base_from_map_qt(ex, ey, yaw, 0.01 * k, pitch=0.02)
-            mo, mr = o.update(ex, ey, refmod.tf2_matrix(q, t)), r.update(ex, ey, q, t)
-            assert mo == mr, k
-            moved_any += mr
-            assert np.array_equal(o.position(), r.position())
-            assert_layers(o, r, ("ground", "groundpatch"), f"roll {k}")
+            moved = m.update(ex, ey, q, t)
+            moved_any += bool(moved)
+            rec.check(f"roll {k}: moved", moved)
+            rec.check(f"roll {k}: position", m.position())
+            check_layers(rec, m, ("ground", "groundpatch"), f"roll {k}")
             push_below_ground(pts, 1500, 600 + k)
-        scan_both(o, r, pts, org, 0.01 * k, f"stream scan {k}")
+        scan(rec, m, pts, org, 0.01 * k, f"stream scan {k}")
     assert moved_any >= 8
 
 
-def test_large_jump_clears_the_map():
-    """A pose jump of more than the map length drops the whole map (grid_map::move -> clearAll + one full region)."""
-    o, r = pair(33.0, 0.33)
+def large_jump_clears_the_map(rec, make):
+    m = new_map(rec, make, 33.0, 0.33)
     scene = synth.make_scene(seed=10, n_boxes=8, rmin=4.0, rmax=14.0)
     pts, org = synth.lidar_scan(scene, beams=24, az_steps=256, seed=1)
-    scan_both(o, r, pts, org, 0.0, "before jump")
+    scan(rec, m, pts, org, 0.0, "before jump")
     q, t = refmod.base_from_map_qt(100.0, -70.0, 0.3, 0.2, pitch=0.01)
-    assert o.update(100.0, -70.0, refmod.tf2_matrix(q, t)) == r.update(100.0, -70.0, q, t) == 1
-    assert np.array_equal(o.position(), r.position())
-    assert_layers(o, r, ("ground", "groundpatch"), "after jump")
+    assert m.update(100.0, -70.0, q, t) == 1
+    rec.check("jump: position", m.position())
+    check_layers(rec, m, ("ground", "groundpatch"), "after jump")
 
 
-@pytest.mark.parametrize("seed", range(8))
-def test_random_geometry_and_config(seed):
-    """Seeded random geometries (integer map lengths: GroundSegmentation::init takes the dimension as size_t) and
-    configurations, two or three scans with a roll in between."""
+def _draw_geometry(rng):
+    return float(rng.integers(24, 70)), float(np.float32(rng.uniform(0.2, 0.6)))
+
+
+def random_geometry_and_config(rec, make, seed):
     rng = np.random.default_rng(9000 + seed)
-    while True:
-        dim = float(rng.integers(24, 70))
-        res = float(np.float32(rng.uniform(0.2, 0.6)))
-        try:
-            refmod.Reference(dim, res)
-        except ValueError:
-            continue
-        break
+
+    def draws_until_accepted():
+        """GroundSegmentation::init takes the map length as size_t: the reference refuses some geometries."""
+        probe = np.random.default_rng(9000 + seed)
+        for k in range(1, 1000):
+            try:
+                refmod.Reference(*_draw_geometry(probe))
+            except ValueError:
+                continue
+            return k
+
+    for _ in range(int(rec.given("geometry draws", draws_until_accepted))):
+        dim, res = _draw_geometry(rng)
     cfg = dict(point_count_cell_variance_threshold=int(rng.integers(0, 30)), max_ring=int(rng.integers(10, 1024)),
                distance_factor=float(rng.uniform(0.0, 0.001)), minimum_distance_factor=float(rng.uniform(1e-4, 0.002)),
                miminum_point_height_threshold=float(rng.uniform(0.1, 0.6)),
@@ -158,7 +161,7 @@ def test_random_geometry_and_config(seed):
                occupied_cells_decrease_factor=float(rng.uniform(1.5, 20.0)),
                occupied_cells_point_count_factor=float(rng.uniform(2.0, 40.0)),
                min_outlier_detection_ground_confidence=float(rng.uniform(0.2, 3.0)))
-    o, r = pair(dim, res, **cfg)
+    m = new_map(rec, make, dim, res, **cfg)
     half = 0.5 * dim
     scene = synth.make_scene(seed=seed, n_boxes=10, rmin=3.0, rmax=0.8 * half)
     ex = ey = 0.0
@@ -169,57 +172,120 @@ def test_random_geometry_and_config(seed):
         pts, org = synth.lidar_scan(scene, (ex, ey), yaw, beams=32, az_steps=512, seed=seed * 10 + k)
         if k:
             q, t = refmod.base_from_map_qt(ex, ey, yaw, 0.05 * k, pitch=float(rng.uniform(-0.03, 0.03)))
-            assert o.update(ex, ey, refmod.tf2_matrix(q, t)) == r.update(ex, ey, q, t)
-            assert np.array_equal(o.position(), r.position())
+            rec.check(f"scan {k}: moved", m.update(ex, ey, q, t))
+            rec.check(f"scan {k}: position", m.position())
             push_below_ground(pts, 400, seed + k)
-        scan_both(o, r, pts, org, 0.05 * k, f"random {seed} dim {dim} res {res} scan {k}")
+        scan(rec, m, pts, org, 0.05 * k, f"random {seed} dim {dim} res {res} scan {k}")
+
+
+def geometry_primitives(rec, make):
+    m = new_map(rec, make, 33.0, 0.33)
+    rng = np.random.default_rng(4)
+
+    def check(ctx):
+        c = m.position()
+        xs = np.concatenate([rng.uniform(-20, 20, 400) + c[0], c[0] + 0.5 * 33.0 + np.array([-1e-9, 0.0, 1e-9]),
+                             c[0] - 0.5 * 33.0 + np.array([-1e-9, 0.0, 1e-9])])
+        ys = np.concatenate([rng.uniform(-20, 20, 400) + c[1], c[1] + rng.uniform(-16, 16, 6)])
+        rows = []
+        for x, y in zip(xs, ys):
+            for fx, fy in ((float(np.float32(x)), float(np.float32(y))), (float(x), float(y))):
+                i, j, inside = m.grid_index(fx, fy)
+                rows.append((i, j, 1) if inside else (0, 0, 0))   # the index of an outside position is not defined
+        rec.check(f"{ctx}: grid_index", np.array(rows))
+        ij = rng.integers(0, m.n, (50, 2))
+        rec.check(f"{ctx}: cell_position", np.array([m.cell_position(int(i), int(j)) for i, j in ij]))
+
+    check("start")
+    q, t = refmod.base_from_map_qt(3.21, -1.77, 0.1, 0.0)
+    assert m.update(3.21, -1.77, q, t) == 1
+    check("moved")
+
+
+def single_phase_calls(rec, make):
+    m = new_map(rec, make, 33.0, 0.33)
+    rng = np.random.default_rng(12)
+    G = rng.normal(0.0, 0.5, (m.n, m.n)).astype(np.float32)
+    Cf = rng.uniform(0.0, 1.0, (m.n, m.n)).astype(np.float32)
+    Cf[rng.uniform(size=Cf.shape) < 0.5] = 0.0
+    m.set_layer("ground", G)
+    m.set_layer("groundpatch", Cf)
+    for x, y in ((5, 7), (48, 49), (49, 49), (1, 1), (97, 97), (60, 12)):
+        m.interpolate_cell(x, y)
+    check_layers(rec, m, ("ground", "groundpatch"), "interpolate_cell")
+    m.spiral(0.25)
+    check_layers(rec, m, ("ground", "groundpatch"), "spiral")
+
+
+SCENARIOS = {
+    "expected_points_table": expected_points_table,
+    "cfg1_cfg2_64_beam_300": cfg1_cfg2_64_beam_300,
+    "cfg3_128_beam_600": cfg3_128_beam_600,
+    "cfg4_four_lidar_364": cfg4_four_lidar_364,
+    "rolling_stream_with_outliers": rolling_stream_with_outliers,
+    "large_jump_clears_the_map": large_jump_clears_the_map,
+    **{f"random_geometry_and_config_{s}": (lambda rec, make, s=s: random_geometry_and_config(rec, make, s)) for s in range(8)},
+    "geometry_primitives": geometry_primitives,
+    "single_phase_calls": single_phase_calls,
+}
+
+
+def against_reference(name):
+    rec = ReferenceRecord(name)
+    SCENARIOS[name](rec, Port)
+    rec.finish()
+
+
+def test_expected_points_table():
+    against_reference("expected_points_table")
+
+
+def test_cfg1_cfg2_64_beam_300():
+    """configs[0]/[1]: ~120 k points, 300 x 300 @ 0.33 m; three scans so that the prior is non-trivial."""
+    against_reference("cfg1_cfg2_64_beam_300")
+
+
+def test_cfg3_128_beam_600():
+    """configs[2]: ~240 k points, 600 x 600 @ 0.2 m."""
+    against_reference("cfg3_128_beam_600")
+
+
+def test_cfg4_four_lidar_364():
+    """configs[3]: four 64-beam sensors, ~480 k points, the reference's own 364 x 364 map."""
+    against_reference("cfg4_four_lidar_364")
+
+
+def test_rolling_stream_with_outliers():
+    """12 scans: ego moves, yaws, the base frame is pitched (position-dependent seeding of exposed cells), points
+    pushed below the ground (outlier ray-march against the rolled prior).  Map position, moved flag, the rolled prior and
+    every layer after every scan must agree."""
+    against_reference("rolling_stream_with_outliers")
+
+
+def test_large_jump_clears_the_map():
+    """A pose jump of more than the map length drops the whole map (grid_map::move -> clearAll + one full region)."""
+    against_reference("large_jump_clears_the_map")
+
+
+@pytest.mark.parametrize("seed", range(8))
+def test_random_geometry_and_config(seed):
+    """Seeded random geometries (integer map lengths: GroundSegmentation::init takes the dimension as size_t) and
+    configurations, two or three scans with a roll in between."""
+    against_reference(f"random_geometry_and_config_{seed}")
 
 
 def test_geometry_primitives_agree():
     """grid_map index <-> position arithmetic of the port (oracle/gridmap_semantics.hpp) against the CPU GridMap the
     reference was compiled with, on random and on edge positions, before and after a move."""
-    o, r = pair(33.0, 0.33)
-    rng = np.random.default_rng(4)
-
-    def check():
-        c = o.position()
-        xs = np.concatenate([rng.uniform(-20, 20, 400) + c[0], c[0] + 0.5 * 33.0 + np.array([-1e-9, 0.0, 1e-9]),
-                             c[0] - 0.5 * 33.0 + np.array([-1e-9, 0.0, 1e-9])])
-        ys = np.concatenate([rng.uniform(-20, 20, 400) + c[1], c[1] + rng.uniform(-16, 16, 6)])
-        for x, y in zip(xs, ys):
-            for fx, fy in ((float(np.float32(x)), float(np.float32(y))), (float(x), float(y))):
-                io, ir = o.grid_index(fx, fy), r.grid_index(fx, fy)
-                assert io[2] == ir[2]
-                if ir[2]:
-                    assert io == ir, (fx, fy, io, ir)
-        for i, j in rng.integers(0, o.n, (50, 2)):
-            assert np.array_equal(o.cell_position(int(i), int(j)), r.cell_position(int(i), int(j)))
-
-    check()
-    q, t = refmod.base_from_map_qt(3.21, -1.77, 0.1, 0.0)
-    assert o.update(3.21, -1.77, refmod.tf2_matrix(q, t)) == r.update(3.21, -1.77, q, t) == 1
-    check()
+    against_reference("geometry_primitives")
 
 
 def test_single_phase_calls_agree():
     """interpolate_cell and the whole spiral called on their own (public methods, GroundSegmentation.h:56-62)."""
-    o, r = pair(33.0, 0.33)
-    rng = np.random.default_rng(12)
-    G = rng.normal(0.0, 0.5, (o.n, o.n)).astype(np.float32)
-    Cf = rng.uniform(0.0, 1.0, (o.n, o.n)).astype(np.float32)
-    Cf[rng.uniform(size=Cf.shape) < 0.5] = 0.0
-    for m in (o, r):
-        m.set_layer("ground", G)
-        m.set_layer("groundpatch", Cf)
-    for x, y in ((5, 7), (48, 49), (49, 49), (1, 1), (97, 97), (60, 12)):
-        o.interpolate_cell(x, y)
-        r.interpolate_cell(x, y)
-    assert_layers(o, r, ("ground", "groundpatch"), "interpolate_cell")
-    o.spiral(0.25)
-    r.spiral(0.25)
-    assert_layers(o, r, ("ground", "groundpatch"), "spiral")
+    against_reference("single_phase_calls")
 
 
+@pytest.mark.skipif(not refmod.available(), reason="oracle/_ref/libgg_ref.so not built (needs the reference sources)")
 def test_reference_threading_as_shipped_runs():
     """thread_count = 8 (the shipped default) is racy and therefore not a parity target; it must still run and label
     nearly everything like the sequential execution (used for the timing baseline)."""
